@@ -41,6 +41,8 @@ WORKLOADS = {
     '50m4k': (50_000_000, 3840, 2160, 1.5, 0),   # config 4 (city scale, 4K): meant for `LGR_MULTI=shard` on 8 GPUs; not yet run
 }
 CPU_SAMPLE = {'10m': 1_000_000, '100k': 100_000, '1k': 1_000, '50m4k': 1_000_000, 'big300k': 20_000}   # Gaussians in the bounded CPU sample
+DUMP_SAMPLE = 1 << 16      # --dump-outputs: Gaussians and pixels kept per array (at most ~25 MB in all, SH degree 3 included)
+GRAD_NAMES = ('dmeans3D', 'dmeans2D', 'dopacities', 'dscales', 'drotations', 'dcolors', 'dshs')
 
 
 def peaks():
@@ -137,6 +139,30 @@ def morton_order(cam, sc, W, H):
     return {k: v[perm].contiguous() for k, v in sc.items()}
 
 
+def dump_outputs(path, out):
+    """--dump-outputs: the arrays the timed path returned in its last step, one DIR/<name>.npy each (float32 as computed,
+    integer arrays as float64).  Per-Gaussian arrays keep the rows listed in gaussian_index.npy, per-pixel arrays the
+    pixels (row-major) listed in pixel_index.npy: fixed seeded samples of DUMP_SAMPLE each, the same in every run, so that
+    two builds can be compared file by file."""
+    os.makedirs(path, exist_ok=True)
+    rng = np.random.default_rng(0)
+    n, (H, W) = out['radii'].shape[0], out['image'].shape[1:]
+    gi = np.sort(rng.choice(n, min(n, DUMP_SAMPLE), replace=False))
+    pi = np.sort(rng.choice(H * W, min(H * W, DUMP_SAMPLE), replace=False))
+    arrays = {'gaussian_index': gi.astype(np.float64), 'pixel_index': pi.astype(np.float64)}
+    gi_d, pi_d = (torch.from_numpy(a).to(out['image'].device) for a in (gi, pi))
+    for name, t in out.items():
+        if t is None:
+            continue
+        per_pixel = name in ('image', 'point_id_pixel', 'point_weight_pixel')
+        t = t.detach().reshape(-1, H * W)[:, pi_d].squeeze(0) if per_pixel else t.detach()[gi_d]
+        a = t.cpu().numpy()
+        arrays[name] = a.astype(np.float32 if a.dtype == np.float32 else np.float64)
+    assert sum(a.nbytes for a in arrays.values()) <= 64 << 20
+    for name, a in arrays.items():
+        np.save(os.path.join(path, name + '.npy'), a)
+
+
 def pick_cpu_threads(c_oracle, step):
     """The CPU arm gets the team size that is FASTEST on this box: all logical CPUs or one thread per physical core
     (half of them) -- the port is bound by memory and atomics, and SMT siblings slow it down on some hosts.  torchrun
@@ -195,6 +221,9 @@ def main():
     ap.add_argument('--impl', default='ours', choices=['ours', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--no-e2e', action='store_true')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one computed as DIR/<name>.npy (rank 0: the image and '
+                         'gradients of its band and Gaussians under N > 1; seeded samples of large arrays)')
     ap.add_argument('--order', default='random', choices=['random', 'morton'],
                     help='order of the synthetic Gaussians in memory: random (SURVEY 8d, the default and the reported metric) or '
                          'sorted along a Morton curve of their screen position (spatially coherent, like tree-ordered LoG data)')
@@ -219,6 +248,8 @@ def main():
     if world > 1:
         dist.init_process_group('nccl', device_id=dev)
     assert world == args.gpus or world == 1, (world, args.gpus)
+    if args.dump_outputs and world > 1 and os.environ.get('LGR_MULTI', 'shard') != 'shard':
+        raise SystemExit('bench.py: --dump-outputs covers one GPU and shard mode; band mode returns packed gradient rows')
 
     n, W, H, r, deg = WORKLOADS[args.workload]
     cam, sc, G = make_inputs(args.workload)
@@ -272,12 +303,12 @@ def main():
                                                      filter_mode=LGR_FILTER_MAX, want_aux=True)
             if record:
                 ev[1].record()
-            g = shard.backward(st, dG)          # sweep + return, barrier, gather + per-Gaussian backward
+            g, pw, _ = shard.backward(st, dG)          # sweep + return, barrier, gather + per-Gaussian backward
             if record:
                 ev[2].record()
                 ev[3].record()
                 phase_ev.append(ev)
-            return g
+            return dict(image=img, radii=radii, point_id_pixel=pid, point_weight_pixel=pwp, point_weight=pw, **dict(zip(GRAD_NAMES, g)))
         if world > 1:      # band mode: owner-grouped id lists, packed gradient rows, one all-to-all to the owner ranks
             ev = [torch.cuda.Event(enable_timing=True) for _ in range(4)]
             ev[0].record()
@@ -302,7 +333,7 @@ def main():
             stats['state'] = st
         if st.max_tile_len is not None:
             stats['D'], stats['D_stock'], stats['maxlen'], stats['visible'] = st.num_instances, st.stock_instances, st.max_tile_len, st.num_visible
-        return g
+        return dict(image=img, radii=radii, point_id_pixel=pid, point_weight_pixel=pwp, point_weight=pw, **dict(zip(GRAD_NAMES, g)))
 
     def barrier():
         torch.cuda.synchronize()
@@ -354,9 +385,11 @@ def main():
         if graph is not None:
             graph.replay()
         else:
-            step_resident()
+            last = step_resident()
     e1.record()
     barrier()
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, g_static if graph is not None else last)
     clk = clocks.stop() if rank == 0 else None
     ms_total = e0.elapsed_time(e1)
     t = torch.tensor([ms_total], device=dev)

@@ -331,12 +331,15 @@ def test_recorded_subtile_bits_do_not_change_the_backward(built, monkeypatch, si
     sc = f32_scene(O.make_scene(n, W, H, r, seed=41))
     G = O.make_cotangent(3, H, W)
     monkeypatch.setattr(R, 'CONTRIB_BITS', False)
-    a = run_gpu(cam, sc, G)
+    a, a2 = run_gpu(cam, sc, G), run_gpu(cam, sc, G)
     monkeypatch.setattr(R, 'CONTRIB_BITS', True)
-    b = run_gpu(cam, sc, G)
+    b, b2 = run_gpu(cam, sc, G), run_gpu(cam, sc, G)
     assert torch.equal(a['image'], b['image'])
     for k in ['dmeans3D', 'dmeans2D', 'dopacities', 'dscales', 'drotations', 'dcolors']:
-        assert rel(b[k], a[k]) < 2e-6, (k, rel(b[k], a[k]))
+        # the blend backward accumulates per-Gaussian gradients with float atomics, so two runs of the SAME path differ in
+        # the last bits (most in dscales, where the chain rule cancels): the bound also covers twice that measured spread
+        spread = max(rel(a2[k], a[k]), rel(b2[k], b[k]))
+        assert rel(b[k], a[k]) < max(2e-6, 2 * spread), (k, rel(b[k], a[k]), spread)
 
 
 @pytest.mark.gpu

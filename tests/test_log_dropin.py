@@ -1,350 +1,230 @@
-"""CPU, build container only (skipped where /root/reference is absent, e.g. on the GPU box): LoG's own
-`LoG/render/renderer.py` imports and runs UNMODIFIED with `dropin/` on the path, binds to this repo's classes for
-both flavours (renderer.py:1, 99-105), builds the rasteriser through `BaseRender.prepare` (:57-78), and its
-`render()` (:117-153) reaches our `GaussianRasterizer.forward` with exactly the keyword set it passes."""
-import os
-import sys
+"""CPU: LoG's own code against this repository's drop-in modules, replayed from tests/golden/reference_log_dropin.npz.
 
+The golden file records what LoG's `LoG/render/renderer.py` and `LoG/model/*`, run UNMODIFIED with `dropin/` on the path
+and this repository's kernels on the CPU SIMT emulation, did with the drop-in: the class each module name LoG imports
+binds to (renderer.py:1, 99-105), the settings `BaseRender.prepare` builds (:57-78), every keyword set `render()`
+(:117-153) passes to `GaussianRasterizer.forward`, the image cotangent LoG's loss sent back, LoG's own
+`TensorTree.traverse` results and LoG's own `SparseOptimizer.step` results (generator: tests/golden/make_dropin_golden.py,
+which needs a LoG checkout).  Here the recorded calls are replayed against the current code: the rasteriser against the
+fp64 oracle, the fused tree walk and the fused sparse Adam against LoG's recorded results."""
+import importlib
+import os
+import types
+
+import numpy as np
 import pytest
 import torch
 
-REF = '/root/reference'
-pytestmark = pytest.mark.skipif(not os.path.isdir(os.path.join(REF, 'LoG')), reason='reference tree not present')
+from oracle import c_oracle, torch_dense as O
+from util import device, rel
+
+GOLD = np.load(os.path.join(os.path.dirname(__file__), 'golden', 'reference_log_dropin.npz'))
+TENSOR_FIELDS = ('bg', 'viewmatrix', 'projmatrix', 'campos')
 
 
-@pytest.fixture(scope='module')
-def renderer_module():
-    cv2 = pytest.importorskip('cv2')  # noqa: F841  (renderer.py imports it)
-    sys.path.insert(0, REF)
-    try:
-        import LoG.render.renderer as R
-    finally:
-        sys.path.remove(REF)
-    return R
+def settings(p, dev):
+    from log_b200 import GaussianRasterizationSettings
+    s = {}
+    for f in GaussianRasterizationSettings._fields:
+        v = GOLD[f'{p}settings/{f}']
+        s[f] = torch.from_numpy(v).to(dev) if f in TENSOR_FIELDS else v.item()
+    return GaussianRasterizationSettings(**s)
 
 
-def camera():
-    return {'FoVx': 1.0, 'FoVy': 0.8, 'image_height': 48, 'image_width': 64, 'world_view_transform': torch.eye(4),
-            'full_proj_transform': torch.eye(4), 'camera_center': torch.zeros(3), 'K': torch.eye(3)}
+def oracle_camera(p):
+    s = settings(p, 'cpu')
+    cam = O.make_camera(s.image_width, s.image_height)
+    return cam._replace(tanfovx=s.tanfovx, tanfovy=s.tanfovy, scale_modifier=s.scale_modifier, sh_degree=s.sh_degree,
+                        **{f: getattr(s, f).double() for f in TENSOR_FIELDS})
 
 
-def test_reference_renderer_binds_to_dropin(renderer_module):
-    R = renderer_module
+def call_names(p, kind):
+    return sorted(k[len(p + kind) + 1:] for k in GOLD.files if k.startswith(p + kind + '/'))
+
+
+def replay(p, dev, tensors=None):
+    """Call the recorded class with the recorded keyword set; `tensors` replaces the recorded tensor values."""
     import log_b200.rasterizer as ours
-    assert R.GaussianRasterizer is ours.GaussianRasterizer                      # `from diff_gaussian_rasterization_wodilate import`
-    R.NaiveRendererAndLoss(use_origin_render=True)
-    assert R.BaseRender.GaussianRasterizer is ours.StockGaussianRasterizer      # `from diff_gaussian_rasterization import`
-    R.NaiveRendererAndLoss(use_origin_render=False)
-    assert R.BaseRender.GaussianRasterizer is ours.GaussianRasterizer
-    rast = R.BaseRender.prepare(camera(), torch.zeros(3))
-    s = rast.raster_settings
+    tensors = tensors or {k: torch.from_numpy(GOLD[f'{p}kw/{k}']) for k in call_names(p, 'kw')}
+    kw = {k: v.to(dev).requires_grad_(bool(GOLD[f'{p}requires_grad/{k}'])) for k, v in tensors.items()}
+    call = dict(kw, **{k: None for k in GOLD[p + 'none']}, **{k: GOLD[f'{p}flag/{k}'].item() for k in call_names(p, 'flag')})
+    rast = getattr(ours, str(GOLD[p + 'class']))(settings(p, dev))
+    out = rast(**call)
+    assert len(out) == int(GOLD[p + 'num_out'])
+    return out, kw
+
+
+def filter_mode(p):
+    if str(GOLD[p + 'class']) == 'StockGaussianRasterizer':
+        return c_oracle.FILTER_ADD
+    return c_oracle.FILTER_NONE if (p + 'flag/use_filter' in GOLD.files and not GOLD[p + 'flag/use_filter']) else c_oracle.FILTER_MAX
+
+
+def check_against_oracle(p, out, kw, G, image_bound=1e-4, grad_bound=2e-4):
+    """The replayed call's outputs and (with cotangent G) the gradients returned into LoG's tensors vs the fp64 oracle."""
+    d = {k: v.detach().cpu().double() for k, v in kw.items()}
+    ref = c_oracle.render(oracle_camera(p), d['means3D'], d['opacities'], d['scales'], d['rotations'], colors_precomp=d['colors_precomp'],
+                          filter_mode=filter_mode(p), dL_dimage=None if G is None else G.double(), dtype=np.float64)
+    assert rel(out[0], ref['image']) < image_bound
+    assert (out[1].cpu().numpy() != ref['radii']).sum() <= 1
+    if len(out) == 5:
+        assert (out[2].cpu().numpy() != ref['point_id_pixel']).sum() <= 2
+        assert rel(out[4], ref['point_weight']) < 1e-4
+    if G is not None:
+        (out[0] * G.to(out[0].device)).sum().backward()
+        pairs = [(n_, g_) for n_, g_ in (('means2D', 'dmeans2D'), ('means3D', 'dmeans3D'), ('colors_precomp', 'dcolors'),
+                                         ('opacities', 'dopacities'), ('scales', 'dscales'), ('rotations', 'drotations')) if kw[n_].requires_grad]
+        # LoG initialises isotropic scales, for which d loss / d rotation is exactly zero, and stays near-isotropic: there
+        # fp32 arithmetic itself cannot reach the bound, which becomes twice the fp32 oracle's own error
+        ref32 = c_oracle.render(oracle_camera(p), d['means3D'], d['opacities'], d['scales'], d['rotations'], colors_precomp=d['colors_precomp'],
+                                filter_mode=filter_mode(p), dL_dimage=G.double(), dtype=np.float32)
+        for name, grad in pairs:
+            assert rel(kw[name].grad.reshape(ref[grad].shape), ref[grad]) < max(grad_bound, 2 * rel(ref32[grad], ref[grad])), name
+    return ref
+
+
+def test_reference_renderer_binds_to_dropin():
+    import log_b200.rasterizer as ours
+    for module, cls in zip(GOLD['bind/modules'], GOLD['bind/classes']):
+        m = importlib.import_module(str(module))
+        assert m.GaussianRasterizer is getattr(ours, str(cls))
+        assert m.GaussianRasterizationSettings is ours.GaussianRasterizationSettings
+    assert list(GOLD['bind/classes']) == ['GaussianRasterizer', 'StockGaussianRasterizer']
+    s = settings('bind/', 'cpu')
     assert (s.image_width, s.image_height, s.sh_degree, s.prefiltered, s.debug) == (64, 48, 0, False, False)
     assert abs(s.tanfovx - 0.5463024898) < 1e-6
+    assert ours.GaussianRasterizer(s).raster_settings is s
 
 
-class _Model:
-    """The three attributes renderer.render() touches (renderer.py:118-140, 174)."""
-    training = False
-    visibility_flag = None
-    empty_xyz = torch.zeros((0, 3))
-
-    def get_all(self, camera, rasterizer, **kw):
-        n = 5
-        return {'xyz': torch.rand(n, 3), 'opacity': torch.rand(n, 1), 'colors': torch.rand(n, 3),
-                'scaling': torch.rand(n, 3), 'rotation': torch.nn.functional.normalize(torch.rand(n, 4))}
-
-
-def test_reference_render_reaches_our_forward_with_its_own_kwargs(renderer_module, built):
+def test_reference_render_reaches_our_forward_with_its_own_kwargs(built):
     """CPU tensors: our forward must be reached (no TypeError on the keyword set, including use_filter=False for the
     fork in eval mode, renderer.py:151-152) and must refuse loudly instead of computing on the CPU."""
-    R = renderer_module
     from log_b200._capi import LgrError
-    rr = R.NaiveRendererAndLoss(use_origin_render=False)
-    rast = R.BaseRender.prepare(camera(), torch.zeros(3))
+    p = 'cpu_refusal/call0/'
+    assert GOLD[p + 'flag/use_filter'].item() is False and str(GOLD[p + 'class']) == 'GaussianRasterizer'
     with pytest.raises(LgrError, match='no CPU fallback'):
-        rr.render(camera(), rast, _Model())
+        replay(p, 'cpu')
 
 
 @pytest.mark.parametrize('origin,training', [(False, True), (False, False), (True, True)])
-def test_reference_render_end_to_end_on_the_emulated_backend(renderer_module, emulated_backend, origin, training):
-    """LoG's own render() (renderer.py:117-205), unmodified, with this repo's rasteriser behind it and the kernels running
-    on the CPU SIMT emulation: the image, radii, point_id / point_count / point_weight it returns equal the oracle's for
-    the flavour and filter it selects (fork + filter in training, fork without filter in eval :151-152, stock with
-    use_origin_render), and loss.backward() fills viewspace_points.grad (read at counter.py:40)."""
-    import numpy as np
-    from oracle import c_oracle, torch_dense as O
-    from util import f32_camera, rel
-    R = renderer_module
+def test_reference_render_end_to_end_on_the_emulated_backend(emulated_backend, origin, training):
+    """LoG's render() with this repo's rasteriser behind it, replayed on the CPU SIMT emulation: the flavour and filter it
+    selected (fork + filter in training, fork without filter in eval :151-152, stock with use_origin_render), the image,
+    radii, point_id / point_count (as LoG's renderer derived them) and point_weight equal the oracle's, and the gradient
+    into viewspace_points (read at counter.py:40) is filled."""
+    name = f'render_origin{int(origin)}_training{int(training)}'
+    p = f'{name}/call0/'
     W, H, n = 64, 48, 300
-    cam = f32_camera(O.make_camera(W, H, bg=(0.0, 0.0, 0.0)))
     sc = {k: v.to(torch.float32) for k, v in O.make_scene(n, W, H, 4.0, seed=12).items()}
-    camera = {'FoVx': 2 * np.arctan(cam.tanfovx), 'FoVy': 2 * np.arctan(cam.tanfovy), 'image_height': H, 'image_width': W,
-              'world_view_transform': cam.viewmatrix.float(), 'full_proj_transform': cam.projmatrix.float(),
-              'camera_center': cam.campos.float(), 'K': torch.eye(3)}
-
-    class Model:
-        visibility_flag = None
-        empty_xyz = torch.zeros((0, 3))
-
-        def get_all(self, camera, rasterizer, **kw):
-            self.leaves = {k: v.clone().requires_grad_(True) for k, v in sc.items()}
-            return {'xyz': self.leaves['means3D'], 'opacity': self.leaves['opacities'], 'colors': self.leaves['colors'],
-                    'scaling': self.leaves['scales'], 'rotation': self.leaves['rotations']}
-    model = Model()
-    model.training = training
-    rr = R.NaiveRendererAndLoss(use_origin_render=origin)
-    rast = R.BaseRender.prepare(camera, torch.zeros(3))
-    ret, _ = rr.render(camera, rast, model)
-    fm = c_oracle.FILTER_ADD if origin else (c_oracle.FILTER_MAX if training else c_oracle.FILTER_NONE)
+    tensors = {'means3D': sc['means3D'], 'means2D': torch.zeros(n, 3), 'colors_precomp': sc['colors'], 'opacities': sc['opacities'],
+               'scales': sc['scales'], 'rotations': sc['rotations']}
+    assert sorted(tensors) == call_names(p, 'kw_sum')
+    for k, v in tensors.items():      # the scene LoG was given is the one regenerated here
+        assert tuple(v.shape) == tuple(GOLD[f'{p}kw_shape/{k}']) and abs(float(v.double().sum()) - float(GOLD[f'{p}kw_sum/{k}'])) < 1e-9
+    assert str(GOLD[p + 'class']) == ('StockGaussianRasterizer' if origin else 'GaussianRasterizer')
+    assert filter_mode(p) == (c_oracle.FILTER_ADD if origin else c_oracle.FILTER_MAX if training else c_oracle.FILTER_NONE)
     G = O.make_cotangent(3, H, W).to(torch.float32)
-    d64 = {k: v.to(torch.float64) for k, v in sc.items()}
-    ref = c_oracle.render(cam, d64['means3D'], d64['opacities'], d64['scales'], d64['rotations'], colors_precomp=d64['colors'],
-                          filter_mode=fm, dL_dimage=G.to(torch.float64), dtype=np.float64)
-    assert ret['render'].shape == (3, H, W) and rel(ret['render'], ref['image']) < 1e-4
-    assert (ret['radii'].numpy() != ref['radii']).sum() <= 1
+    out, kw = replay(p, device(), tensors)
+    ref = check_against_oracle(p, out, kw, G)
     if not origin:
         ids, cnt = np.unique(ref['point_id_pixel'], return_counts=True)
         keep = ids >= 0
-        assert (ret['point_id'].numpy() != ids[keep]).sum() <= 2 if ret['point_id'].numel() == keep.sum() else False
-        assert abs(int(ret['point_count'].sum()) - int(cnt[keep].sum())) <= 3
-        assert rel(ret['point_weight'], ref['point_weight']) < 1e-4
-    (ret['render'] * G).sum().backward()
-    assert rel(ret['viewspace_points'].grad, ref['dmeans2D']) < 2e-4
-    assert rel(model.leaves['means3D'].grad, ref['dmeans3D']) < 2e-4
-    assert rel(model.leaves['colors'].grad, ref['dcolors']) < 1e-4
+        pid, pcount = GOLD[f'{name}/ret/point_id'], GOLD[f'{name}/ret/point_count']
+        assert (pid != ids[keep]).sum() <= 2 if len(pid) == keep.sum() else False
+        assert abs(int(pcount.sum()) - int(cnt[keep].sum())) <= 3
+        got_ids, got_cnt = np.unique(out[2].cpu().numpy(), return_counts=True)
+        assert np.array_equal(got_ids[got_ids >= 0], pid) and np.array_equal(got_cnt[got_ids >= 0], pcount)
+    assert float(kw['means2D'].grad.abs().sum()) > 0
+
+
+def walk_objects(p, dev):
+    """Stand-ins for LoG's TensorTree / Gaussian / rasteriser: the attributes log_b200.tree.traverse reads."""
+    max_child, max_level = (int(x) for x in GOLD[p + 'tree_args'])
+    t = lambda k: torch.from_numpy(GOLD[p + k]).to(dev)
+    tree = types.SimpleNamespace(node_index=t('node_index'), tree=t('tree'), max_child=max_child, max_level=max_level)
+    model = types.SimpleNamespace(xyz=t('xyz'), scaling=t('scaling'), rotation=t('rotation'),
+                                  activation=types.SimpleNamespace(scaling_activation=torch.exp))
+    return tree, model, types.SimpleNamespace(raster_settings=settings(p, dev))
+
+
+def check_walk(p_tree, p_query):
+    from log_b200.tree import traverse
+    dev = device()
+    tree, model, rast = walk_objects(p_tree, dev)
+    tree.min_resolution_pixel, max_depth = GOLD[p_query + 'args']
+    got = traverse(tree, model, torch.from_numpy(GOLD[p_query + 'roots']).long().to(dev), rast, max_depth=int(max_depth))
+    assert got.dtype == torch.int64
+    assert np.array_equal(got.cpu().numpy(), GOLD[p_query + 'want']), p_query
+    return got
 
 
 def test_fused_tree_walk_equals_the_reference_traverse_call_path(emulated_backend):
-    """The reference's own `TensorTree.traverse` driving its own `Gaussian.compute_radius` (level_of_gaussian.py:64-93, with
-    dropin/LoG_cuda/compute_radius.py in place of the JIT module, i.e. this repo's lgr_compute_radius underneath) against
-    `log_b200.tree.traverse` on the same objects: identical index tensors, also when many nodes are culled (radius 0)."""
-    import importlib.util
-    import numpy as np
-    from log_b200 import GaussianRasterizationSettings, GaussianRasterizer
-    from log_b200.tree import traverse
-    from oracle import torch_dense as O
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-    spec = importlib.util.spec_from_file_location('LoG.cuda.compute_radius', os.path.join(root, 'dropin', 'LoG_cuda', 'compute_radius.py'))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    saved = sys.modules.get('LoG.cuda.compute_radius')
-    sys.modules['LoG.cuda.compute_radius'] = mod
-    sys.path.insert(0, REF)
-    try:
-        import LoG.model.level_of_gaussian as L
-        from LoG.model.tensor_tree import TensorTree
-    finally:
-        sys.path.remove(REF)
-        if saved is not None:
-            sys.modules['LoG.cuda.compute_radius'] = saved
-    rng = np.random.default_rng(3)
-    cam = O.make_camera(160, 96)
-    settings = GaussianRasterizationSettings(
-        image_height=96, image_width=160, tanfovx=cam.tanfovx, tanfovy=cam.tanfovy, bg=torch.zeros(3), scale_modifier=1.0,
-        viewmatrix=cam.viewmatrix.float(), projmatrix=cam.projmatrix.float(), sh_degree=0, campos=cam.campos.float(),
-        prefiltered=False, debug=False)
-    rast = GaussianRasterizer(settings)
-    for max_child, n_root in ((2, 120), (4, 50)):
-        tree = TensorTree(max_child=max_child, max_level=20)
-        tree.initialize(torch.zeros(n_root, 3))
-        for rd in range(4):
-            leaves = torch.where(tree.is_leaf & (tree.depth == rd))[0]
-            tree.split(leaves[torch.from_numpy(rng.random(len(leaves)) < 0.6)])
-        P = tree.num_points
-        depth = tree.depth.numpy().astype(np.float64)
-        z = rng.uniform(0.5, 10.0, P)
-        g = L.Gaussian()
-        g.xyz = torch.from_numpy(np.stack([rng.uniform(-2.0, 2.0, P) * cam.tanfovx * z, rng.uniform(-2.0, 2.0, P) * cam.tanfovy * z, z], -1)).float()
-        sig = np.exp(rng.normal(np.log(12.0) - 1.0 * depth, 1.0)) / 3.0 * z / (160 / (2 * cam.tanfovx))
-        g.scaling = torch.from_numpy(np.log(sig[:, None] * rng.uniform(0.3, 1.0, (P, 3)))).float()
-        g.rotation = torch.from_numpy(rng.normal(size=(P, 4))).float()
-        roots = torch.where(tree.is_root)[0]
-        for min_px, max_depth in ((3.0, 1000), (6.0, 2), (1.5, 1000)):
-            tree.min_resolution_pixel = min_px
-            want = tree.traverse(g, roots.long(), rast, max_depth=max_depth)
-            got = traverse(tree, g, roots.long(), rast, max_depth=max_depth)
-            r2d = g.compute_radius(want, rast)[1]
-            assert (r2d == 0).sum() > 10                               # culled nodes are part of the case
-            if (torch.abs(r2d[r2d > 0] / min_px - 1) < 1e-4).any():     # a radius within fp32 noise of the threshold: skip it
-                continue
-            assert torch.equal(got, want), (max_child, min_px, max_depth)
+    """LoG's own `TensorTree.traverse` driving its own `Gaussian.compute_radius` (level_of_gaussian.py:64-93, with
+    dropin/LoG_cuda/compute_radius.py underneath) against `log_b200.tree.traverse` on the same objects: identical index
+    tensors, also when many nodes are culled (radius 0)."""
+    nq = GOLD['walk/num_queries']
+    assert len(nq) == 2 and nq.sum() >= 4
+    for t, q in ((t, q) for t in range(len(nq)) for q in range(int(nq[t]))):
+        check_walk(f'walk/tree{t}/', f'walk/tree{t}/q{q}/')
 
 
-def _miniature_log(monkeypatch, densify=None):
-    """LoG's own model / renderer / batch for a 64x48 view of 300 points (see test_log_training_loop_in_miniature)."""
-    import importlib.util
-    import types
-    import numpy as np
-    from oracle import c_oracle, torch_dense as O
-    from util import rel
-    root = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-
-    def dist2(x):                                  # mean squared distance to the 3 nearest neighbours, as distCUDA2
-        d = torch.cdist(x, x)
-        d.fill_diagonal_(float('inf'))
-        return (d.topk(3, largest=False).values ** 2).mean(-1)
-    knn, knn_c = types.ModuleType('simple_knn'), types.ModuleType('simple_knn._C')
-    knn_c.distCUDA2, knn._C = dist2, knn_c
-    monkeypatch.setitem(sys.modules, 'simple_knn', knn)
-    monkeypatch.setitem(sys.modules, 'simple_knn._C', knn_c)
-    monkeypatch.setattr(torch.Tensor, 'cuda', lambda self, *a, **k: self)
-    spec = importlib.util.spec_from_file_location('LoG.cuda.compute_radius', os.path.join(root, 'dropin', 'LoG_cuda', 'compute_radius.py'))
-    mod = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(mod)
-    monkeypatch.setitem(sys.modules, 'LoG.cuda.compute_radius', mod)
-    monkeypatch.syspath_prepend(REF)
-    import LoG.model.level_of_gaussian as L
-    import LoG.render.renderer as R
-
-    class AD(dict):
-        __getattr__ = dict.__getitem__
-
-    rng = np.random.default_rng(0)
-    W, H, n = 64, 48, 300
-    cam = O.make_camera(W, H)
-    z = rng.uniform(2, 6, n)
-    xyz = np.stack([rng.uniform(-1, 1, n) * cam.tanfovx * z, rng.uniform(-1, 1, n) * cam.tanfovy * z, z], -1).astype(np.float32)
-    colors = rng.uniform(0, 1, (n, 3)).astype(np.float32)
-    model = L.LoG(gaussian=dict(init_ply=dict(filename={'xyz': xyz, 'colors': colors}, scale3d=1., init_opacity=0.5), sh_degree=1, xyz_scale=1.),
-                  tree=AD(max_child=2, max_level=5),
-                  optimizer=AD(optimize_keys=['xyz', 'colors', 'scaling', 'opacity', 'rotation', 'shs'], opt_all_levels=True,
-                               lr_dict=dict(xyz=0.00016, xyz_final=0.0000016, xyz_scale=1., colors=0.0025, shs=0.000125, scaling=0.005,
-                                            opacity=0.05, rotation=0.001, max_steps=100)),
-                  densify_and_remove=AD(dict(upgrade_sh_iter=10, densify_from_iter=1, densify_every_iter=1, upgrade_repeat=50), **(densify or {})),
-                  use_view_correction=False)
-    model.base_iter = 1
-    model.training_setup()
-    model.train()
-    rend = R.NaiveRendererAndLoss(split='train')
-    batch = {'camera': {'camera_center': cam.campos.float()[None], 'world_view_transform': cam.viewmatrix.float()[None],
-                        'full_proj_transform': cam.projmatrix.float()[None], 'image_width': torch.tensor([W]), 'image_height': torch.tensor([H]),
-                        'FoVx': torch.tensor([2 * np.arctan(cam.tanfovx)]), 'FoVy': torch.tensor([2 * np.arctan(cam.tanfovy)]),
-                        'K': torch.eye(3)[None], 'R': torch.eye(3)[None], 'T': torch.zeros(1, 3, 1)},
-             'image': torch.rand(1, H, W, 3, generator=torch.Generator().manual_seed(1)), 'index': torch.tensor([0])}
-    return model, rend, batch, cam
+def check_loop_calls(scenario):
+    """Every kept rasteriser call of a LoG training loop, with the cotangent LoG's loss sent back, against the oracle."""
+    for i in GOLD[f'{scenario}/calls_kept']:
+        p = f'{scenario}/call{i}/'
+        assert str(GOLD[p + 'class']) == 'GaussianRasterizer' and filter_mode(p) == c_oracle.FILTER_MAX
+        out, kw = replay(p, device())
+        check_against_oracle(p, out, kw, torch.from_numpy(GOLD[p + 'grad_image']).float())
 
 
-def test_log_training_loop_in_miniature(emulated_backend, monkeypatch):
+def test_log_training_loop_in_miniature(emulated_backend):
     """BASELINE config 3 in miniature: LoG's OWN classes -- `LoG` / `GaussianPoint` / `TensorTree` / `Counter` /
-    `SparseOptimizer` (LoG/model/level_of_gaussian.py) and `NaiveRendererAndLoss` (LoG/render/renderer.py) -- drive a few
-    training iterations exactly as `Trainer.training_step` does (LoG/utils/trainer.py:144-166: render, loss.backward(),
-    update_by_output, step) with this repo's rasteriser and compute_radius behind them (kernels on the CPU emulation).
-    Checked: the first loss equals LoG's own loss applied to the ORACLE's image of the same parameters, the loss goes down,
-    the parameters move, the counters fill.  Test-only stand-ins: simple_knn.distCUDA2 (a CUDA-only third party, used once
-    for the initial scales) and Tensor.cuda()."""
-    import numpy as np
-    from oracle import c_oracle, torch_dense as O
-    from util import rel
-    model, rend, batch, cam = _miniature_log(monkeypatch)
-    g = model.gaussian
-    act = g.activation
-    start = {k: getattr(g, k).clone() for k in ('xyz', 'scaling', 'opacity', 'rotation', 'colors')}
-    ref = c_oracle.render(cam, g.xyz.double(), act.opacity_activation(g.opacity).double(), act.scaling_activation(g.scaling).double(),
-                          act.rotation_activation(g.rotation).double(), colors_precomp=(g.colors * O.C0 + 0.5).double(),
-                          filter_mode=c_oracle.FILTER_MAX, dtype=np.float64)
-    losses = []
-    for it in range(5):
-        model.clear()
-        out = rend(batch, model)                       # Trainer.training_step, trainer.py:144-166
-        out['loss'].backward()
-        model.update_by_output(out)
-        model.step()
-        losses.append(float(out['loss'].detach()))
-        if it == 0:
-            first = {}
-            rend.calculate_loss(batch['image'].permute(0, 3, 1, 2), torch.from_numpy(ref['image']).float()[None], first)
-            assert abs(losses[0] - float(first['loss'])) < 1e-5 * max(1.0, abs(losses[0]))
-            assert rel(out['render'][0], ref['image']) < 1e-4
-    assert all(b < a for a, b in zip(losses, losses[1:])), losses
-    assert all(float((getattr(g, k) - start[k]).abs().max()) > 0 for k in start)       # SparseOptimizer moved every parameter group
-    assert int(model.counter.visible_count.sum()) > 0 and float(model.counter.weights_max.max()) > 0
-    assert int(model.optimizer.global_steps.item()) == 5
+    `SparseOptimizer` (LoG/model/level_of_gaussian.py) and `NaiveRendererAndLoss` (LoG/render/renderer.py) -- drove five
+    training iterations as `Trainer.training_step` does (LoG/utils/trainer.py:144-166: render, loss.backward(),
+    update_by_output, step) with this repo's rasteriser behind them; when recorded, the loss fell at every step and the
+    first loss equalled LoG's loss of the ORACLE's image.  Replayed: the last iteration's rasteriser call, image and every
+    gradient LoG received (with the cotangent LoG's loss sent back, stored at half precision), against the oracle."""
+    assert list(GOLD['loop/calls_kept']) == [4] and int(GOLD['loop/num_calls']) == 5
+    check_loop_calls('loop')
 
 
-def test_log_training_loop_with_tree_nodes_and_the_fused_walk(emulated_backend, monkeypatch):
+def test_log_training_loop_with_tree_nodes_and_the_fused_walk(emulated_backend):
     """The same loop taken into LoG's depth stage: `upgrade_tree`, `update_depth_stage` (LoG's own Splitter creates child
     nodes), then training continues through `LoG.prepare` -> `render_to_check` -> `TensorTree.traverse`
-    (level_of_gaussian.py:223-257).  `tree.traverse` is replaced by `log_b200.tree.traverse`; in every call the fused walk
-    returns exactly the tensor LoG's own traverse returns, and the loss keeps falling."""
-    from log_b200.tree import traverse as fused
-    model, rend, batch, cam = _miniature_log(monkeypatch, densify=dict(
-        split_grad_thres=0.0, radius2d_thres=0, min_steps_split=0, remove_weights_thres=0.005, max_split_points=20000,
-        sort_method='radii', scaling_decay=0.9))
-
-    def train(iters):
-        out_losses = []
-        for _ in range(iters):
-            model.clear()
-            out = rend(batch, model)
-            out['loss'].backward()
-            model.update_by_output(out)
-            model.step()
-            out_losses.append(float(out['loss'].detach()))
-        return out_losses, out
-    train(3)
-    model.set_stage('depth')
-    model.upgrade_tree()                       # level_of_gaussian.py:527-533
-    train(3)
-    model.update_depth_stage(10)               # :454-525 -> tree.split_and_remove + Splitter
-    assert model.tree.num_nodes > 0 and model.num_points > 300
-    reference_traverse, agree = model.tree.traverse, []
-
-    def both(g, root_index, rasterizer, max_depth=1000):
-        want = reference_traverse(g, root_index, rasterizer, max_depth=max_depth)
-        got = fused(model.tree, g, root_index, rasterizer, max_depth=max_depth)
-        agree.append(bool(torch.equal(got, want)))
-        return got
-    model.tree.traverse = both
-    losses, out = train(4)
-    assert agree == [True] * 4
-    assert losses[-1] < losses[0], losses
-    assert out['visibility_flag'][0]['index_node'].numel() > 0       # parents and leaves are both in play
+    (level_of_gaussian.py:223-257).  `log_b200.tree.traverse` returns exactly the tensor LoG's own traverse returned
+    (first and last walk), and the last rasteriser call matches the oracle."""
+    walks = GOLD['deep/walks_kept']
+    assert int(GOLD['deep/num_walks']) == 4 and list(walks) == [0, 3]
+    for w in walks:
+        got = check_walk(f'deep/walk{w}/', f'deep/walk{w}/')
+        assert got.numel() > 0 and int(GOLD[f'deep/walk{w}/node_index'].shape[0]) > 300
+    check_loop_calls('deep')
 
 
-def test_log_training_loop_with_the_fused_sparse_adam(emulated_backend, monkeypatch):
-    """`SparseOptimizer.step` (LoG/model/sparse_optimizer.py:163-196: gather state, `_single_tensor_adam`, scatter back) replaced
-    by one `sparse_adam_step_` per parameter, as INTEGRATION.md describes: after five iterations of LoG's own training step
-    every parameter tensor and both Adam moments equal the reference optimiser's (fp32 round-off)."""
+def test_log_training_loop_with_the_fused_sparse_adam(emulated_backend):
+    """`SparseOptimizer.step` (LoG/model/sparse_optimizer.py:163-196: gather state, `_single_tensor_adam`, scatter back)
+    replaced by one `sparse_adam_step_` per parameter, as INTEGRATION.md describes: for each of LoG's five steps and each
+    parameter group, the rows of the parameter and both Adam moments equal LoG's own optimiser's (a seeded sample of the
+    visible rows is stored; the rows left out are zero and must stay zero)."""
     from log_b200.optim import sparse_adam_step_
-    from util import rel
-
-    def run(fused):
-        model, rend, batch, cam = _miniature_log(monkeypatch)
-        if fused:
-            def step(self, gaussian, index, params, flag_vis):
-                self.global_steps += 1
-                index = index[flag_vis].contiguous()
-                for key, param in params.items():
-                    if param.grad is None:
-                        continue
-                    if key == 'xyz':
-                        lr = self.xyz_scheduler_args(self.global_steps.item())
-                        self.xyz_lr = lr
-                    elif key == 'scaling':
-                        lr = self.scaling_scheduler_args(self.global_steps.item())
-                    else:
-                        lr = self.lr_dict[key]
-                    sparse_adam_step_(getattr(gaussian, key).data, param.grad[flag_vis].contiguous(), self.exp_avg[key],
-                                      self.exp_avg_sq[key], index, step=int(self.global_steps.item()), lr=lr, eps=1e-15)
-            model.optimizer.step = step.__get__(model.optimizer)
-        for _ in range(5):
-            model.clear()
-            out = rend(batch, model)
-            out['loss'].backward()
-            model.update_by_output(out)
-            model.step()
-        g, o = model.gaussian, model.optimizer
-        state = {k: getattr(g, k).clone() for k in ('xyz', 'scaling', 'opacity', 'rotation', 'colors')}
-        state.update({f'm_{k}': o.exp_avg[k].clone() for k in ('xyz', 'scaling', 'opacity')})
-        state.update({f'v_{k}': o.exp_avg_sq[k].clone() for k in ('xyz', 'scaling', 'opacity')})
-        return state, float(out['loss'].detach())
-    ref, loss_ref = run(False)
-    got, loss_got = run(True)
-    assert abs(loss_ref - loss_got) < 1e-6
-    for k in ref:
-        # LoG initialises isotropic scales, for which d loss / d rotation is exactly zero: the rotation gradient is float
-        # noise, Adam turns noise into +-lr steps, and the two optimisers' differently rounded noise drifts apart (1e-4).
-        # Once the scales have taken their first +-lr steps they are no longer isotropic, so the drifted rotations feed
-        # the scale gradient (and its Adam moments) at the same 1e-4 level; the scales themselves still agree exactly.
-        loose = k in ('rotation', 'm_scaling', 'v_scaling')
-        assert rel(got[k], ref[k]) < (2e-3 if loose else 2e-6), (k, rel(got[k], ref[k]))
+    dev = device()
+    assert int(GOLD['loop/num_steps']) == 5
+    for s in range(5):
+        keys = list(GOLD[f'loop/step{s}/keys'])
+        assert {'xyz', 'scaling', 'opacity', 'rotation', 'colors'} <= set(keys)
+        for key in keys:
+            p = f'loop/step{s}/{key}/'
+            step, lr, n = GOLD[p + 'hyper']
+            rows = torch.from_numpy(GOLD[p + 'rows']).to(dev)
+            full = {}
+            for k in ('param', 'm', 'v'):
+                a = GOLD[f'{p}{k}_in']
+                full[k] = torch.zeros((int(n),) + a.shape[1:], dtype=torch.float32, device=dev)
+                full[k][rows] = torch.from_numpy(a).to(dev)
+            sparse_adam_step_(full['param'], torch.from_numpy(GOLD[p + 'grad']).to(dev), full['m'], full['v'], rows,
+                              step=int(step), lr=float(lr), eps=1e-15)
+            rest = torch.ones(int(n), dtype=torch.bool, device=dev)
+            rest[rows] = False
+            for k in ('param', 'm', 'v'):
+                assert rel(full[k][rows], GOLD[f'{p}{k}_out']) < 2e-6, (s, key, k)
+                assert not full[k][rest].any(), (s, key, k)
