@@ -9,7 +9,7 @@
 // Backward: the same front-to-back walk (closed form of the published recurrence, see below).  Per contributing hit every
 // lane publishes two scalars; every 8 hits the warp contracts them against fixed per-pixel weights (pixel-coordinate
 // moments and cotangent-weighted sums) on the tensor cores (mma.sync m16n8k8, split TF32 = fp32 accuracy); the moments
-// become gradients once per staged splat, then 3 vector atomics per splat.  With View::contrib the forward records which
+// become gradients right after each contraction, then 3 vector atomics per (warp, hit).  With View::contrib the forward records which
 // sub-tiles composited each list entry and the backward (REC) walks exactly those pairs, stopping every pixel after its
 // last contributor (the forward's n_contrib) instead of re-testing boxes and transmittances.
 #include "lgr_common.cuh"
@@ -89,9 +89,6 @@ __device__ __forceinline__ uint32_t pin_reg(uint32_t v) {
 }
 __device__ __forceinline__ void red_shared_max_u32(uint32_t addr, unsigned v) {
   asm volatile("red.shared.max.u32 [%0], %1;" ::"r"(addr), "r"(v) : "memory");
-}
-__device__ __forceinline__ void red_shared_add_f32(uint32_t addr, float v) {
-  asm volatile("red.shared.add.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
 }
 __device__ __forceinline__ void sts_f32(uint32_t addr, float v) {
   asm volatile("st.shared.f32 [%0], %1;" ::"r"(addr), "f"(v) : "memory");
@@ -286,20 +283,21 @@ blend_fwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
 //
 // Reduction over the warp's pixels.  Every one of the 9 per-splat outputs is a FIXED-weight linear functional of two
 // per-lane scalars of the hit, wG = dL/dG * G and w = alpha * T:
-//     M00, M10, M01, M20, M11, M02 = sum_l wG_l * {1, u, v, u^2, uv, v^2}_l      (u, v: tile-centred pixel coordinates)
+//     M00, M10, M01, M20, M11, M02 = sum_l wG_l * {1, u, v, u^2, uv, v^2}_l      (u, v: pixel coordinates about the warp's sub-tile centre)
 //     C0, C1, C2                   = sum_l w_l * dL/dC_{0,1,2; l}
 // i.e. a [hits x 32] x [32 x 9] contraction.  Each lane publishes (wG, w) of a contributing hit as one row element of two
 // [8 hits][32 pixels] shared-memory blocks; when 8 hits are pending (or the batch ends) the warp runs the contraction
 // on the tensor cores: A (16 rows = 8 wG rows + 8 w rows) straight from the blocks with ldmatrix, B = the weights (moment
-// weights are small half-integers and their products: exact in TF32; the cotangent weights are split hi + lo once per
+// weights are quarter-integers, |u^2| <= 12.25: exact in TF32; the cotangent weights are split hi + lo once per
 // kernel), every A value split hi + lo, fp32 accumulation -- 8 + 12 mma.m16n8k8 per 8 hits, error ~2^-20 relative.
-// The D fragments (hit x output) are added into per-splat shared accumulators.  The moments are turned
-// into d/dmean2D, d/dconic, d/dopacity once per staged splat when the batch is flushed (X = splat centre, same
-// coordinates):
+// Right after the contraction the 4 lanes of hit g's fragment group gather its 9 sums with 4 shuffles, turn the moments
+// into d/dmean2D, d/dconic, d/dopacity (X = splat centre in the same coordinates):
 //     sum wG dx = X M00 - M10,   sum wG dx^2 = X^2 M00 - 2 X M10 + M20,   sum wG dx dy = XY M00 - X M01 - Y M10 + M11 ...
+// and add them into dsplat with one vector atomic each (fire-and-forget RED, no shared-memory accumulators).
 constexpr int HITS = 8;          // hits per contraction (half the m of mma.m16n8k8: 8 wG rows + 8 w rows)
 constexpr int XROW = 36;         // floats per published row: 32 pixels + 4 pad, so the 8 rows of an ldmatrix block hit 8 bank groups
-constexpr int BWD_SMEM = BATCH * 48 + BATCH * 36 + (BLEND_THREADS / 32) * (2 * HITS * XROW + 192 + 192) * 4 + BATCH;
+constexpr int BWD_SMEM = BATCH * 48 + (BLEND_THREADS / 32) * (2 * HITS * XROW + 192 + 192) * 4 + BATCH;
+static_assert(BWD_SMEM <= 48 * 1024, "the backward launches without the large-shared-memory opt-in");
 
 // REC: the forward recorded (View::contrib) which sub-tiles composited each list entry and (View::last_contrib = its
 // n_contrib output) where every pixel's last contributor sits; the sweep then meets exactly the contributing (sub-tile,
@@ -311,24 +309,23 @@ blend_bwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
                  const float* __restrict__ dL_dimage, float* __restrict__ dsplat) {
   extern __shared__ float4 smem_f4[];
   float4* s_rec = smem_f4;                                                        // [BATCH * 3]
-  float* s_g = reinterpret_cast<float*>(s_rec + BATCH * 3);                       // [BATCH * 9]
-  float* s_x = s_g + BATCH * 9;                                                   // per warp: wG[8][36] | w[8][36]
-  float* s_cw = s_x + (BLEND_THREADS / 32) * 2 * HITS * XROW;                     // per warp: cotangent weights, hi/lo, A-fragment order
-  float* s_mw = s_cw + (BLEND_THREADS / 32) * 192;                                // per warp: moment weights, A-fragment order
+  float* s_x = reinterpret_cast<float*>(s_rec + BATCH * 3);                       // per warp: wG[8][36] | w[8][36]
+  float* s_cw = s_x + (BLEND_THREADS / 32) * 2 * HITS * XROW;                     // per warp: cotangent weights, B-fragment order
+  float* s_mw = s_cw + (BLEND_THREADS / 32) * 192;                                // per warp: moment weights, B-fragment order
   unsigned char* s_bits = reinterpret_cast<unsigned char*>(s_mw + (BLEND_THREADS / 32) * 192);      // [BATCH]
   const int tile = blockIdx.x, tid = threadIdx.x, lane = tid & 31, warp = tid >> 5;
   const SubTile st = make_subtile(v, tile, lane, warp);
   const float pxf = (float)st.x, pyf = (float)st.y;
   const float tx0 = (float)((tile % v.gx) * TILE), ty0 = (float)((v.row0 + tile / v.gx) * TILE);
   const int beg = tile_start[tile], len = tile_start[tile + 1] - beg;
-  const uint32_t s_g_addr = pin_reg(smem_u32(s_g));
   const uint32_t s_rec_addr = pin_reg(smem_u32(s_rec));
   const uint32_t xg_addr = pin_reg(smem_u32(s_x) + (uint32_t)warp * (2 * HITS * XROW * 4));
   const uint32_t xlane_addr = pin_reg(xg_addr + 4u * (uint32_t)lane);
   // ldmatrix row address of this lane: row lane%8 of block lane/8; blocks = (wG, chunk 2s), (w, chunk 2s), (wG, chunk 2s+1), (w, chunk 2s+1)
   const uint32_t xrow = pin_reg(xg_addr + (uint32_t)(lane & 7) * (XROW * 4) + (uint32_t)((lane >> 3) & 1) * (HITS * XROW * 4) +
                                 (uint32_t)(lane >> 4) * 16u);
-  const float tcx = tx0 + 7.5f, tcy = ty0 + 7.5f;
+  const float ucx = (warp & 1) * 8 + 3.5f, ucy = (warp >> 1) * 4 + 1.5f;   // moment origin: this warp's sub-tile centre
+  const float tcx = tx0 + ucx, tcy = ty0 + ucy;
   const int g = lane >> 2, t = lane & 3;        // mma fragment coordinates of this lane
 
   float Rd = 0.f, dp0 = 0.f, dp1 = 0.f, dp2 = 0.f;
@@ -339,26 +336,30 @@ blend_bwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
     Rd = image[pix] * dp0 + image[HW + pix] * dp1 + image[2 * HW + pix] * dp2;
     if (REC) last = v.last_contrib[pix];
   }
-  // B fragments of the moment weights, per warp in shared memory: s_mw[((g*4 + t)*4 + s)*2 + {0,1}] = weight of output g at
-  // the pixel of k-step s with k = t (column t, row s of the sub-tile) / k = t + 4 (column t + 4).  |values| <= 56.25 in
-  // steps of 0.25: exact in TF32.
-  const uint32_t mw_addr = pin_reg(smem_u32(s_mw) + (uint32_t)warp * (192 * 4) + (uint32_t)((min(g, 5) * 4 + t) * 32));
+  // B fragments of the weights, per warp in shared memory, lane-major per k-step so that the load of k-step s reads
+  // consecutive addresses (one LDS.64 / LDS.128 over 192 bytes).  Only the lanes of the used columns have an entry:
+  // g < 6 (lanes 0..23) for the moments, g < 3 (lanes 0..11) for the cotangents.  The other lanes load the last entry
+  // again (a broadcast, no extra wavefront, no branch): it lands in D columns that are never read (moments 6, 7 of t = 3;
+  // colour columns >= 3).
+  // Moments: s_mw[(s*24 + lane)*2 + {0,1}] = weight of output g at the pixel of k-step s with k = t (column t, row s of the
+  // sub-tile) / k = t + 4 (column t + 4).  Multiples of 0.25, |values| <= 12.25: exact in TF32.
+  const uint32_t mw_addr = pin_reg(smem_u32(s_mw) + (uint32_t)warp * (192 * 4) + (uint32_t)min(lane, 23) * 8u);
   for (int k = lane; k < 192; k += 32) {
-    const int which = k & 1, s_ = (k >> 1) & 3, t_ = (k >> 3) & 3, g_ = k >> 5;
-    const float u = (float)((warp & 1) * 8 + t_ + 4 * which) - 7.5f, vv = (float)((warp >> 1) * 4 + s_) - 7.5f;
+    const int which = k & 1, s_ = (k >> 1) / 24, l_ = (k >> 1) % 24, t_ = l_ & 3, g_ = l_ >> 2;
+    const float u = (float)((warp & 1) * 8 + t_ + 4 * which) - ucx, vv = (float)((warp >> 1) * 4 + s_) - ucy;
     const float f = g_ == 0 ? 1.f : g_ == 1 ? u : g_ == 2 ? vv : g_ == 3 ? u * u : g_ == 4 ? u * vv : vv * vv;
     s_mw[warp * 192 + k] = f;
   }
-  // B fragments of the cotangent weights (columns 0..2 = channel): s_cw[((c*4 + t)*4 + s)*4 + {0,1,2,3}] = hi(k=t), hi(k=t+4), lo(k=t), lo(k=t+4)
-  const uint32_t cw_addr = pin_reg(smem_u32(s_cw) + (uint32_t)warp * (192 * 4) + (uint32_t)((min(g, 2) * 4 + t) * 64));
+  // Cotangents (columns 0..2 = channel): s_cw[(s*12 + c*4 + t)*4 + {0,1,2,3}] = hi(k=t), hi(k=t+4), lo(k=t), lo(k=t+4)
+  const uint32_t cw_addr = pin_reg(smem_u32(s_cw) + (uint32_t)warp * (192 * 4) + (uint32_t)min(lane, 11) * 16u);
   {
     float* cw = s_cw + warp * 192;
     const int col = lane & 7, s = lane >> 3, tt = col & 3, which = col >> 2;
     const float dpc[3] = {dp0, dp1, dp2};
 #pragma unroll
     for (int c = 0; c < 3; c++) {
-      cw[((c * 4 + tt) * 4 + s) * 4 + which] = dpc[c];                  // read as trunc(x) by the tensor core
-      cw[((c * 4 + tt) * 4 + s) * 4 + 2 + which] = tf32_lo(dpc[c]);
+      cw[(s * 12 + c * 4 + tt) * 4 + which] = dpc[c];                  // read as trunc(x) by the tensor core
+      cw[(s * 12 + c * 4 + tt) * 4 + 2 + which] = tf32_lo(dpc[c]);
     }
   }
   __syncwarp();
@@ -367,15 +368,13 @@ blend_bwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
   int done = st.inside ? (REC ? (last == 0) : 0) : 1;
   int id_next = tid < len ? sorted_ids[beg + tid] : -1;
 
-  // Two barriers per batch, as in the forward: thread tid stages, flushes and re-stages only slot tid (record, hit bits and
-  // the nine accumulators of that splat).
+  // Two barriers per batch: A (the batch is staged) and B (every warp has left the walk, so slot tid may be re-staged).
+  // Thread tid stages only slot tid (record and hit bits).
   int base = 0, cnt = min(BATCH, len);
   auto stage = [&]() {
     if (tid < cnt) {
       // with View::contrib: walk exactly the (sub-tile, splat) pairs that composited something in the forward
       stage_splat(s_rec, s_bits, tid, splat, id_next, tx0, ty0, REC ? v.contrib + beg + base + tid : nullptr);
-#pragma unroll
-      for (int k = 0; k < 9; k++) s_g[tid * 9 + k] = 0.f;
     } else {
       s_bits[tid] = 0;
     }
@@ -485,10 +484,8 @@ blend_bwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
             ldsm_x4(xrow + 32u * s, a0, a1, a2, a3);
             const uint32_t l0 = __float_as_uint(tf32_lo(__uint_as_float(a0))), l1 = __float_as_uint(tf32_lo(__uint_as_float(a1)));
             const uint32_t l2 = __float_as_uint(tf32_lo(__uint_as_float(a2))), l3 = __float_as_uint(tf32_lo(__uint_as_float(a3)));
-            float2 bm = make_float2(0.f, 0.f);
-            float4 bc = make_float4(0.f, 0.f, 0.f, 0.f);
-            if (g < 6) bm = lds_f2(mw_addr + 8u * s);
-            if (g < 3) bc = lds_f4(cw_addr + 16u * s);
+            const float2 bm = lds_f2(mw_addr + 192u * s);
+            const float4 bc = lds_f4(cw_addr + 192u * s);
             mma_tf32(d0, d1, z0, z1, a0, a1, a2, a3, __float_as_uint(bm.x), __float_as_uint(bm.y));
             mma_tf32(y0, y1, d2, d3, a0, a1, a2, a3, __float_as_uint(bc.x), __float_as_uint(bc.y));
             mma_tf32(d0, d1, z0, z1, l0, l1, l2, l3, __float_as_uint(bm.x), __float_as_uint(bm.y));
@@ -496,11 +493,40 @@ blend_bwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
             mma_tf32(y0, y1, d2, d3, a0, a1, a2, a3, __float_as_uint(bc.z), __float_as_uint(bc.w));
           }
           // lane (g, t): d0/d1 = moments 2t, 2t+1 of hit g (t < 3) ; d2/d3 = colour sums 2t, 2t+1 of hit g (t = 0: 0, 1; t = 1: 2)
-          const uint32_t acc = s_g_addr + 36u * (uint32_t)__shfl_sync(FULL, my_e, g);
-          if (g < pend) {
-            if (t < 3) { red_shared_add_f32(acc + 8u * t, d0); red_shared_add_f32(acc + 8u * t + 4u, d1); }
-            if (t < 2) red_shared_add_f32(acc + 24u + 8u * t, d2);
-            if (t == 0) red_shared_add_f32(acc + 28u, d3);
+          const int e = __shfl_sync(FULL, my_e, g);
+          // Gather within the lane group, 4 shuffles: t = 0 (d/dmean2D, d/dconic_xy) needs M01, M20 (from t = 1) and M11
+          // (t = 2); t = 1 (d/dconic_z, d/dopacity, d/drg) needs M00, C0, C1 (t = 0) and M02 (t = 2); t = 2 (d/db) needs
+          // C2 (t = 1).  Source lane of x2: t = 0 <- 2, 1 <- 0, 2 <- 1.
+          const int src = (lane & ~3) | ((0x3102 >> (4 * t)) & 3);
+          const float x0 = __shfl_xor_sync(FULL, d0, 1);                      // t = 0: M01   t = 1: M00
+          const float x1 = __shfl_down_sync(FULL, d1, 1);                     // t = 0: M20   t = 1: M02
+          const float x2 = __shfl_sync(FULL, t == 2 ? d0 : d2, src);          // t = 0: M11   t = 1: C0   t = 2: C2
+          const float x3 = __shfl_xor_sync(FULL, d3, 1);                      //              t = 1: C1
+          if (g < pend && t < 3) {
+            const uint32_t rec = s_rec_addr + 48u * (uint32_t)e;
+            const float4 r0 = lds_f4(rec);                                    // (px, py, conic_x', conic_y')
+            const float2 r1 = lds_f2(rec + 16u);                              // (conic_z', opacity)
+            float* dst = dsplat + (int64_t)__float_as_int(lds_f2(rec + 40u).y) * LGR_GRAD_FLOATS;
+            const float X = r0.x - tcx, Y = r0.y - tcy;
+            float4 part;                               // float4 t of the splat's gradient row: one vector atomic per lane
+            if (t == 0) {
+              const float M00 = d0, M10 = d1, M01 = x0, M20 = x1, M11 = x2;
+              const float Sx = fmaf(X, M00, -M10), Sy = fmaf(Y, M00, -M01);                       // sum wG dx, sum wG dy
+              const float Sxx = fmaf(X, fmaf(X, M00, -2.f * M10), M20);                           // sum wG dx^2
+              const float Sxy = fmaf(X, fmaf(Y, M00, -M01), fmaf(-Y, M10, M11));                  // sum wG dx dy
+              part.x = -(r0.z * Sx + r0.w * Sy);       // d/dpx  (x log2e: the conic in the record is pre-scaled)
+              part.y = -(r1.x * Sy + r0.w * Sx);       // d/dpy  (x log2e)
+              part.z = -0.5f * Sxx;                    // d/dconic_x
+              part.w = -Sxy;                           // d/dconic_y
+            } else if (t == 1) {
+              const float M00 = x0, M01 = d0, M02 = x1;
+              part.x = -0.5f * fmaf(Y, fmaf(Y, M00, -2.f * M01), M02);                             // d/dconic_z = -sum wG dy^2 / 2
+              part.y = M00 * rcp_approx(r1.y);         // d/dopacity = sum G dL/dalpha = sum wG / o
+              part.z = x2; part.w = x3;                // d/dr, d/dg
+            } else {
+              part = make_float4(x2, 0.f, 0.f, 0.f);   // d/db; the row's 3 padding floats stay 0
+            }
+            atomicAdd(reinterpret_cast<float4*>(dst) + t, part);
           }
           __syncwarp();
           pend = 0;
@@ -509,34 +535,6 @@ blend_bwd_kernel(View v, const int32_t* __restrict__ tile_start, const int32_t* 
       }
     }
     const int all_done = __syncthreads_and(done);      // B: every warp has left the walk
-    if (tid < cnt) {
-      const float* m = s_g + tid * 9;
-      const float M00 = m[0], M10 = m[1], M01 = m[2], M20 = m[3], M11 = m[4], M02 = m[5];
-      const bool nz = (M00 != 0.f) | (M10 != 0.f) | (M01 != 0.f) | (M20 != 0.f) | (M11 != 0.f) | (M02 != 0.f) |
-                      (m[6] != 0.f) | (m[7] != 0.f) | (m[8] != 0.f);
-      if (nz) {
-        const float4 r0 = s_rec[3 * tid];
-        const float2 r1 = *reinterpret_cast<const float2*>(&s_rec[3 * tid + 1]);
-        const int id = __float_as_int(s_rec[3 * tid + 2].w);
-        const float X = r0.x - tcx, Y = r0.y - tcy;
-        const float Sx = fmaf(X, M00, -M10), Sy = fmaf(Y, M00, -M01);                       // sum wG dx, sum wG dy
-        const float Sxx = fmaf(X, fmaf(X, M00, -2.f * M10), M20);                           // sum wG dx^2
-        const float Syy = fmaf(Y, fmaf(Y, M00, -2.f * M01), M02);
-        const float Sxy = fmaf(X, fmaf(Y, M00, -M01), fmaf(-Y, M10, M11));                  // sum wG dx dy
-        float4 a, b;
-        a.x = -(r0.z * Sx + r0.w * Sy);          // d/dpx  (x log2e: the conic in the record is pre-scaled)
-        a.y = -(r1.x * Sy + r0.w * Sx);          // d/dpy  (x log2e)
-        a.z = -0.5f * Sxx;                       // d/dconic_x
-        a.w = -Sxy;                              // d/dconic_y
-        b.x = -0.5f * Syy;                       // d/dconic_z
-        b.y = M00 / r1.y;                        // d/dopacity = sum G dL/dalpha = sum wG / o
-        b.z = m[6]; b.w = m[7];                  // d/drgb
-        float4* dst = reinterpret_cast<float4*>(dsplat + (int64_t)id * LGR_GRAD_FLOATS);
-        atomicAdd(dst, a);
-        atomicAdd(dst + 1, b);
-        atomicAdd(reinterpret_cast<float*>(dst + 2), m[8]);
-      }
-    }
     base += BATCH;
     if (all_done || base >= len) break;
     cnt = min(BATCH, len - base);
@@ -569,11 +567,7 @@ int launch_blend_bwd(const View& v, const int32_t* tile_start, const int32_t* so
                      const float* image, const float* dL_dimage, float* dsplat, cudaStream_t st) {
   const int ntiles = v.gx * (v.row1 - v.row0);
   if (ntiles <= 0) return 0;
-  // > 48 KB of dynamic shared memory needs the opt-in; the attribute is per device and cheap to set, so set it every time
   const bool rec = v.contrib != nullptr && v.last_contrib != nullptr;
-  cudaError_t e = rec ? cudaFuncSetAttribute(blend_bwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM)
-                      : cudaFuncSetAttribute(blend_bwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, BWD_SMEM);
-  if (e != cudaSuccess) return (int)e;
   ProfScope ps(K_BLEND_BWD, st);
   if (rec) blend_bwd_kernel<true><<<ntiles, BLEND_THREADS, BWD_SMEM, st>>>(v, tile_start, sorted_ids, splat, image, dL_dimage, dsplat);
   else blend_bwd_kernel<false><<<ntiles, BLEND_THREADS, BWD_SMEM, st>>>(v, tile_start, sorted_ids, splat, image, dL_dimage, dsplat);

@@ -10,7 +10,7 @@ LIB = os.path.join(ROOT, 'log_b200', '_lib', 'liblog_b200_raster.so')
 PATS = collections.OrderedDict([
     ('HMMA (mma.sync tf32)', r'\bHMMA\.'), ('LDSM (ldmatrix)', r'\bLDSM'), ('UTC*MMA / LDTM (tcgen05)', r'UTC\w*MMA|LDTM'),
     ('UBLKCP / UTMA (bulk / tensor copies)', r'UBLKCP|UTMA'), ('REDUX', r'\bREDUX'), ('VOTE', r'\bVOTE'), ('MATCH', r'\bMATCH'),
-    ('SHFL', r'\bSHFL'), ('ATOMS / REDS (shared)', r'\bATOMS|\bREDS'), ('ATOMG (returning)', r'\bATOMG'), ('RED (global)', r'\bRED\.'),
+    ('SHFL', r'\bSHFL'), ('ATOMS / REDS (shared)', r'\bATOMS|\bREDS'), ('ATOMG (returning)', r'\bATOMG'), ('RED (global)', r'\bREDG?\.E\.'),
     ('MUFU.EX2', r'MUFU\.EX2'), ('BAR', r'\bBAR\.'), ('LDG.128', r'LDG\.E\.(\w+\.)*128'), ('STG.128', r'STG\.E\.(\w+\.)*128'),
     ('CCTL (L2 prefetch)', r'\bCCTL')])
 
